@@ -61,7 +61,31 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subconfigs", action="store_true", help="skip the configs[1] / configs[2] sub-records")
     ap.add_argument("--no-roofline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy "
+                         "(float32; rank 0's shard when several GPUs run), so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has nothing to dump")
+    return args
+
+
+DUMP_BYTES = 63_000_000   # all dumped arrays together, kept under 64 MB with the .npy headers
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor of `arrays` as <dirname>/<name>.npy in float32.  When together they exceed DUMP_BYTES,
+    each is replaced by tests.util.seeded_sample of its share of that budget: the same positions on every run."""
+    from tests.util import seeded_sample
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values()) * 4
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if total > DUMP_BYTES:
+            a = seeded_sample(a, a.numel() * DUMP_BYTES // total)
+        np.save(os.path.join(dirname, name + ".npy"), a.numpy())
 
 
 def load_peaks():
@@ -415,12 +439,17 @@ def run_ours(args, hp, sd):
         ms = shard.max_over_ranks(float(e0.elapsed_time(e1)), dev)
         return ms, clocks
 
+    last = {}
+
     def device_loop(n):
         for _ in range(n):
-            step_device()
+            last["wave"] = step_device()
 
     sampler = ClockSampler(local) if rank == 0 else None
     ms, clocks = timed(device_loop, args.steps, args.warmup, sampler)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+    del last
     n_launch = launches[0]
     total_samples = float(world * B * L * args.steps)
     value = total_samples / (ms * 1e-3)
@@ -576,8 +605,9 @@ def bench_generator(args, hp, dev, lib, peaks):
     return out
 
 
-def bench_whisper(args, dev, lib, peaks):
-    """BASELINE configs[2]: truncated Whisper large-v2 encoder (24 blocks), 16 x 30 s log-mel per step."""
+def bench_whisper(args, dev, lib, peaks, dump=None):
+    """BASELINE configs[2]: truncated Whisper large-v2 encoder (24 blocks), 16 x 30 s log-mel per step.
+    `dump`, when given, receives the PPG of the last timed step under "ppg"."""
     from whisper_vits_svc_b200 import synth, whisper_infer
     ck = synth.whisper_checkpoint(seed=1234)
     enc = whisper_infer.WhisperB200(ck, dev).encoder
@@ -586,7 +616,9 @@ def bench_whisper(args, dev, lib, peaks):
     g = torch.Generator().manual_seed(0)
     mel = torch.randn(B, 80, n, generator=g).clamp(-1, 1.5)
     mel_d = mel.to(dev)
-    ms = timed_region(lambda: enc(mel_d), steps, max(args.warmup, 3), dev) / steps
+    last = {} if dump is None else dump
+    ms = timed_region(lambda: last.update(ppg=enc(mel_d)), steps, max(args.warmup, 3), dev) / steps
+    del last
     pipe = E2EPipeline(dev, {"mel": mel.pin_memory()}, (B, 1500, 1280), lambda x: enc(x["mel"]))
     pipe.run(1)
     torch.cuda.synchronize(dev)
@@ -641,9 +673,10 @@ def bench_whisper(args, dev, lib, peaks):
     return out
 
 
-def bench_hubert(args, dev, lib, peaks):
+def bench_hubert(args, dev, lib, peaks, dump=None):
     """SURVEY.md §8f-2 (not a BASELINE config): HuBERT-Soft units, 16 x 20 s chunks of 16 kHz audio per step
-    (hubert/inference.py:30-33 chunk size) -> [16, 1000, 256]."""
+    (hubert/inference.py:30-33 chunk size) -> [16, 1000, 256].  `dump`, when given, receives the units of the
+    last timed step under "units"."""
     from whisper_vits_svc_b200 import hubert_infer, synth
     sd = synth.hubert_checkpoint(1234)
     model = hubert_infer.HubertSoftB200(sd, dev)
@@ -653,7 +686,9 @@ def bench_hubert(args, dev, lib, peaks):
     wav = torch.randn(B, n, generator=g) * 0.1
     wav_d = wav.to(dev)
     T = model.frames(n)
-    ms = timed_region(lambda: model.units(wav_d), steps, max(args.warmup, 3), dev) / steps
+    last = {} if dump is None else dump
+    ms = timed_region(lambda: last.update(units=model.units(wav_d)), steps, max(args.warmup, 3), dev) / steps
+    del last
     pipe = E2EPipeline(dev, {"wav": wav.pin_memory()}, (B, T, 256), lambda x: model.units(x["wav"]))
     pipe.run(1)
     torch.cuda.synchronize(dev)
@@ -698,7 +733,10 @@ def run_whisper(args):
     assert torch.cuda.is_available()
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", 0)))
     torch.cuda.set_device(dev)
-    out = (bench_hubert if args.workload == "hubert" else bench_whisper)(args, dev, _lib.load(), load_peaks())
+    dump = {}
+    out = (bench_hubert if args.workload == "hubert" else bench_whisper)(args, dev, _lib.load(), load_peaks(), dump)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump)
     out.update({"n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "data": "synthetic"})
     print(json.dumps(out), flush=True)

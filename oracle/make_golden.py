@@ -177,6 +177,44 @@ def hubert_case(name):
     print(name, tuple(units.shape), "units rms %.3f" % units.pow(2).mean().sqrt().item(), "oracle-vs-reference max abs", err)
 
 
+LIVE_WHISPER = [(dict(n_audio_state=256, n_audio_head=4, n_audio_layer=8), 2, 120),
+                (dict(n_audio_state=384, n_audio_head=6, n_audio_layer=4), 1, 77)]
+LIVE_THREADS = 8   # CPU matmuls split their sums by thread count: the tests run the oracle with this many too
+
+
+def live_case(name, hp):
+    """What the *_reference_live tests of tests/test_oracle_cpu.py compare the oracle with: the reference's outputs
+    on their inputs (each as tests.util.seeded_sample plus `<key>_shape`), the number of Whisper encoder blocks the
+    loader keeps, the layout (names, shapes as "d0,d1,...") and alias-filter taps of a fresh SynthesizerInfer, and
+    the intra-op thread count the outputs were computed with."""
+    from tests.util import seeded_sample
+    torch.set_num_threads(LIVE_THREADS)
+    out, arrays = {}, {"threads": np.int64(LIVE_THREADS)}
+    sd = synth.svc_state_dict(hp, 1234)
+    d = make_inputs(77, 2, 33, hp, ragged=True)
+    with torch.no_grad(), FeedRNG([d["rand_ini"]], [d["noise"], d["eps"]]):
+        m = ref_model(hp, sd)
+        out["infer_source"] = m.pitch2source(d["pit"])
+        out["infer_wave"] = m.inference(d["ppg"], d["vec"], d["pit"], d["spk"], d["ppg_l"], out["infer_source"])
+    for over, B, n in LIVE_WHISPER:
+        key = f"whisper_d{over['n_audio_state']}_b{B}_n{n}"
+        model = ref_whisper(synth.whisper_checkpoint(whisper_dims(over), seed=5))
+        with torch.no_grad():
+            out[key] = model.encoder(whisper_mel(6, B, n))
+        arrays[key + "_blocks"] = np.int64(len(model.encoder.blocks))
+    out["hubert_b1_n5003"] = ref_hubert(synth.hubert_checkpoint(7)).units(hubert_wav(8, 1, 5003))
+    for k, v in out.items():
+        arrays[k] = seeded_sample(v).numpy()
+        arrays[k + "_shape"] = np.array(v.shape, dtype=np.int64)
+    fresh = ref_import.import_synthesizer()(hp.data.filter_length // 2 + 1, hp.data.segment_size // hp.data.hop_length,
+                                             ref_import.to_attr(hp)).state_dict()
+    arrays["sd_keys"] = np.array(list(fresh))
+    arrays["sd_shapes"] = np.array([",".join(map(str, v.shape)) for v in fresh.values()])
+    arrays["sd_filter"] = fresh["dec.activation_post.upsample.filter"].numpy()
+    np.savez_compressed(os.path.join(GOLDEN, name + ".npz"), **arrays)
+    print(name, {k: tuple(v.shape) for k, v in out.items()})
+
+
 if __name__ == "__main__":
     os.makedirs(GOLDEN, exist_ok=True)
     hp = hparams.load_hparams(os.path.join(ROOT, "configs", "base.yaml"))
@@ -189,3 +227,4 @@ if __name__ == "__main__":
         whisper_case(name)
     for name in HUBERT_CASES:
         hubert_case(name)
+    live_case("reference_live", hp)

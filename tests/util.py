@@ -39,6 +39,18 @@ def make_inputs(seed: int, B: int, T: int, hp, ragged: bool = False, gen_only: b
     return d
 
 
+def seeded_sample(x, k: int = 8192):
+    """A fixed, seeded sample of k values of x (flattened; all of x when it has at most k): the same positions
+    for every x of one size, so that samples of two runs compare value for value.  Golden fixtures and
+    `bench.py --dump-outputs` keep large outputs small this way.  The positions are random so that no stride
+    of the output's layout (channels, up-sampling phases) is left out."""
+    flat = torch.as_tensor(x).reshape(-1)
+    if flat.numel() <= k:
+        return flat
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:k].sort().values
+    return flat[idx]
+
+
 def max_abs(a, b):
     return float((torch.as_tensor(a).float().cpu() - torch.as_tensor(b).float().cpu()).abs().max())
 
