@@ -235,12 +235,8 @@ def amp_block(sd: SD, p: str, x: torch.Tensor, k: int, dilations=(1, 3, 5)) -> t
     return x
 
 
-def generator(sd: SD, hp, spk, x, source, stages: Optional[dict] = None):
-    """Generator.inference, vits_decoder/generator.py:175-200 (+ SpeakerAdapter :36-47)."""
-    rates = list(hp.gen.upsample_rates)
-    ksz = list(hp.gen.upsample_kernel_sizes)
-    rk = list(hp.gen.resblock_kernel_sizes)
-    rd = [tuple(d) for d in hp.gen.resblock_dilation_sizes]
+def gen_pre(sd: SD, spk, x):
+    """SpeakerAdapter (vits_decoder/generator.py:36-47) + conv_pre + Mish (generator.py:178-181)."""
     # SpeakerAdapter: biased variance, eps inside the sqrt
     xt = x.transpose(1, -1)
     mean = xt.mean(dim=-1, keepdim=True)
@@ -251,30 +247,54 @@ def generator(sd: SD, hp, spk, x, source, stages: Optional[dict] = None):
     y = y * scale.unsqueeze(1) + bias.unsqueeze(1)
     x = y.transpose(1, -1)
     x = F.conv1d(x, sd["dec.conv_pre.weight"], sd["dec.conv_pre.bias"], padding=3)
-    x = x * torch.tanh(F.softplus(x))
-    if stages is not None:
-        stages["gen_pre"] = x
-    for i, (u, k) in enumerate(zip(rates, ksz)):
-        w = fold_weight_norm(sd, f"dec.ups.{i}")
-        x = F.conv_transpose1d(x, w, sd[f"dec.ups.{i}.bias"], stride=u, padding=(k - u) // 2)
-        nw = sd[f"dec.noise_convs.{i}.weight"]
-        if i + 1 < len(rates):
-            s = int(np.prod(rates[i + 1:]))
-            x = x + F.conv1d(source, nw, sd[f"dec.noise_convs.{i}.bias"], stride=s, padding=s // 2)
-        else:
-            x = x + F.conv1d(source, nw, sd[f"dec.noise_convs.{i}.bias"])
-        if stages is not None:
-            stages[f"gen_up{i}"] = x
-        acc = None
-        for j, kk in enumerate(rk):
-            r = amp_block(sd, f"dec.resblocks.{i * len(rk) + j}", x, kk, rd[j])
-            acc = r if acc is None else acc + r
-        x = acc / len(rk)
-        if stages is not None:
-            stages[f"gen_stage{i}"] = x
+    return x * torch.tanh(F.softplus(x))
+
+
+def gen_up(sd: SD, hp, i: int, x, source):
+    """Up-sampling stage i: ups[i] (ConvTranspose1d) + noise_convs[i](source), generator.py:183-186."""
+    rates = list(hp.gen.upsample_rates)
+    u, k = rates[i], list(hp.gen.upsample_kernel_sizes)[i]
+    w = fold_weight_norm(sd, f"dec.ups.{i}")
+    x = F.conv_transpose1d(x, w, sd[f"dec.ups.{i}.bias"], stride=u, padding=(k - u) // 2)
+    nw = sd[f"dec.noise_convs.{i}.weight"]
+    if i + 1 < len(rates):
+        s = int(np.prod(rates[i + 1:]))
+        return x + F.conv1d(source, nw, sd[f"dec.noise_convs.{i}.bias"], stride=s, padding=s // 2)
+    return x + F.conv1d(source, nw, sd[f"dec.noise_convs.{i}.bias"])
+
+
+def gen_amp_stage(sd: SD, hp, i: int, x):
+    """The mean of stage i's n_res AMP blocks, generator.py:188-194."""
+    rk = list(hp.gen.resblock_kernel_sizes)
+    rd = [tuple(d) for d in hp.gen.resblock_dilation_sizes]
+    acc = None
+    for j, kk in enumerate(rk):
+        r = amp_block(sd, f"dec.resblocks.{i * len(rk) + j}", x, kk, rd[j])
+        acc = r if acc is None else acc + r
+    return acc / len(rk)
+
+
+def gen_post(sd: SD, x):
+    """activation_post + conv_post + tanh, generator.py:196-199."""
     x = snake_alias(sd, "dec.activation_post", x)
     x = F.conv1d(x, sd["dec.conv_post.weight"], None, padding=3)
     return torch.tanh(x)
+
+
+def generator(sd: SD, hp, spk, x, source, stages: Optional[dict] = None):
+    """Generator.inference, vits_decoder/generator.py:175-200 (+ SpeakerAdapter :36-47).
+    Runs in the dtype of its arguments: a float64 state dict and inputs give a float64 generator."""
+    x = gen_pre(sd, spk, x)
+    if stages is not None:
+        stages["gen_pre"] = x
+    for i in range(len(hp.gen.upsample_rates)):
+        x = gen_up(sd, hp, i, x, source)
+        if stages is not None:
+            stages[f"gen_up{i}"] = x
+        x = gen_amp_stage(sd, hp, i, x)
+        if stages is not None:
+            stages[f"gen_stage{i}"] = x
+    return gen_post(sd, x)
 
 
 # --------------------------------------------------------------------------- NSF source
