@@ -127,32 +127,49 @@ def ffn(sd: SD, p: str, x: torch.Tensor, mask: torch.Tensor, k: int = 3):
     return h * mask
 
 
-def prior_encoder(sd: SD, ppg, ppg_l, vec, pit, eps, n_layers=6, stages: Optional[dict] = None):
-    """TextEncoder.forward, vits/models.py:39-52; Encoder.forward attentions.py:60-72.
-    `eps` replaces torch.randn_like(m) at models.py:51."""
-    f0c = f0_to_coarse(pit)
-    x = ppg.transpose(1, -1)
-    mask = sequence_mask(ppg_l, x.shape[2]).unsqueeze(1).to(x.dtype)
-    x = F.conv1d(x, sd["enc_p.pre.weight"], sd["enc_p.pre.bias"], padding=2) * mask
+def enc_front(sd: SD, ppg, vec, pit, mask):
+    """pre + hub + pitch embedding, vits/models.py:40-47, before Encoder.forward's `x * x_mask`.
+    The pitch bin is computed from the float32 pitch whatever the dtype of the rest: the reference reads
+    pitch as a FloatTensor and bins it in float32, and float64 arithmetic puts some pitches in the
+    neighbouring bin."""
+    f0c = f0_to_coarse(pit.float())
+    x = F.conv1d(ppg.transpose(1, -1), sd["enc_p.pre.weight"], sd["enc_p.pre.bias"], padding=2) * mask
     v = F.conv1d(vec.transpose(1, -1), sd["enc_p.hub.weight"], sd["enc_p.hub.bias"], padding=2) * mask
-    x = x + v + F.embedding(f0c, sd["enc_p.pit.weight"]).transpose(1, 2)
-    if stages is not None:
-        stages["enc_front"] = x
+    return x + v + F.embedding(f0c, sd["enc_p.pit.weight"]).transpose(1, 2)
+
+
+def enc_layer(sd: SD, i: int, x, mask):
+    """Encoder layer i (attention + FFN, each with its residual LayerNorm), attentions.py:63-71.
+    Layer 0 expects x already multiplied by the mask (attentions.py:62)."""
+    e = "enc_p.enc."
     attn_mask = mask.unsqueeze(2) * mask.unsqueeze(-1)
-    x = x * mask
-    for i in range(n_layers):
-        e = "enc_p.enc."
-        y = rel_attention(sd, f"{e}attn_layers.{i}", x, attn_mask)
-        x = channel_layer_norm(x + y, sd[f"{e}norm_layers_1.{i}.gamma"], sd[f"{e}norm_layers_1.{i}.beta"])
-        y = ffn(sd, f"{e}ffn_layers.{i}", x, mask)
-        x = channel_layer_norm(x + y, sd[f"{e}norm_layers_2.{i}.gamma"], sd[f"{e}norm_layers_2.{i}.beta"])
-        if stages is not None:
-            stages[f"enc_layer{i}"] = x
+    y = rel_attention(sd, f"{e}attn_layers.{i}", x, attn_mask)
+    x = channel_layer_norm(x + y, sd[f"{e}norm_layers_1.{i}.gamma"], sd[f"{e}norm_layers_1.{i}.beta"])
+    y = ffn(sd, f"{e}ffn_layers.{i}", x, mask)
+    return channel_layer_norm(x + y, sd[f"{e}norm_layers_2.{i}.gamma"], sd[f"{e}norm_layers_2.{i}.beta"])
+
+
+def enc_proj(sd: SD, x, mask, eps):
+    """Encoder's final mask, proj and the reparameterisation, attentions.py:72 + vits/models.py:49-51 -> z_p."""
     x = x * mask
     stats = F.conv1d(x, sd["enc_p.proj.weight"], sd["enc_p.proj.bias"]) * mask
     m, logs = torch.split(stats, stats.shape[1] // 2, dim=1)
-    z_p = (m + eps * torch.exp(logs)) * mask
-    return z_p, mask
+    return (m + eps * torch.exp(logs)) * mask
+
+
+def prior_encoder(sd: SD, ppg, ppg_l, vec, pit, eps, n_layers=6, stages: Optional[dict] = None):
+    """TextEncoder.forward, vits/models.py:39-52; Encoder.forward attentions.py:60-72.
+    `eps` replaces torch.randn_like(m) at models.py:51."""
+    mask = sequence_mask(ppg_l, ppg.shape[1]).unsqueeze(1).to(ppg.dtype)
+    x = enc_front(sd, ppg, vec, pit, mask)
+    if stages is not None:
+        stages["enc_front"] = x
+    x = x * mask
+    for i in range(n_layers):
+        x = enc_layer(sd, i, x, mask)
+        if stages is not None:
+            stages[f"enc_layer{i}"] = x
+    return enc_proj(sd, x, mask, eps), mask
 
 
 # --------------------------------------------------------------------------- flow
@@ -188,12 +205,16 @@ def coupling_reverse(sd: SD, p: str, x, mask, spk):
     return torch.cat([x0, x1], 1)
 
 
+def flow_step(sd: SD, i: int, x, mask, spk):
+    """Flip (modules.py:225-229) then coupling layer i in reverse (`flow.flows.{2i}`)."""
+    return coupling_reverse(sd, f"flow.flows.{2 * i}", torch.flip(x, [1]), mask, spk)
+
+
 def flow_reverse(sd: SD, z_p, mask, spk, n_flows=4, stages: Optional[dict] = None):
     """ResidualCouplingBlock.forward(reverse=True), vits/models.py:89-94: reversed([RCL,Flip]*4)."""
     x = z_p
     for i in reversed(range(n_flows)):
-        x = torch.flip(x, [1])  # Flip, modules.py:225-229
-        x = coupling_reverse(sd, f"flow.flows.{2 * i}", x, mask, spk)
+        x = flow_step(sd, i, x, mask, spk)
         if stages is not None:
             stages[f"flow{i}"] = x
     return x

@@ -57,7 +57,7 @@ import pytest
 import torch
 
 from oracle import svc_oracle as O
-from tests.util import GOLDEN, make_inputs, max_abs
+from tests.util import GOLDEN, launched_kernels, make_inputs, max_abs
 from whisper_vits_svc_b200 import hparams, synth
 
 pytestmark = pytest.mark.gpu
@@ -242,18 +242,6 @@ def test_generator_stage_vs_float64(cfg, B, T, precision):
 
 
 # ------------------------------------------------------------------------------------------------ dispatch
-def _kernel_set(m, c, B, T, hpx):
-    from whisper_vits_svc_b200 import _lib
-    lib = _lib.load()
-    lib.svcb_timing_enable(1)
-    try:
-        run_device(m, c, B, T, hpx)
-        rep = lib.svcb_timing_report().decode()
-    finally:
-        lib.svcb_timing_enable(0)
-    return {line.split()[0] for line in rep.splitlines() if line.strip()}
-
-
 def _amp(prefix, ch, ks=(3, 7, 11), suffix=""):
     return {f"{prefix}_c{ch}k{k}{suffix}" for k in ks}
 
@@ -323,7 +311,7 @@ def test_dispatch_kernel_sets(cfg, precision):
     s2d_link_factor) cannot move a stage to another kernel without the stage table above changing with it."""
     hpx = _hp(cfg)
     B, T = 2, 13
-    got = _kernel_set(_model(cfg, precision), _case(cfg, B, T), B, T, hpx)
+    got = launched_kernels(lambda: run_device(_model(cfg, precision), _case(cfg, B, T), B, T, hpx))
     print(f"\n{cfg} precision {precision}: {sorted(got)}")
     assert got == KERNELS[(cfg, precision)], (f"missing {sorted(KERNELS[(cfg, precision)] - got)}, "
                                               f"unexpected {sorted(got - KERNELS[(cfg, precision)])}")

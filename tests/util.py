@@ -51,6 +51,22 @@ def seeded_sample(x, k: int = 8192):
     return flat[idx]
 
 
+def launched_kernels(fn) -> set:
+    """Names of the kernels the device launches during `fn()`, read from svcb_timing_report with kernel
+    timing switched on for the call."""
+    import torch
+    from whisper_vits_svc_b200 import _lib
+    lib = _lib.load()
+    lib.svcb_timing_enable(1)
+    try:
+        fn()
+        torch.cuda.synchronize()
+        rep = lib.svcb_timing_report().decode()
+    finally:
+        lib.svcb_timing_enable(0)
+    return {line.split()[0] for line in rep.splitlines() if line.strip()}
+
+
 def max_abs(a, b):
     return float((torch.as_tensor(a).float().cpu() - torch.as_tensor(b).float().cpu()).abs().max())
 
